@@ -56,6 +56,52 @@ def traffic_bytes():
     return None, "no ncu summary found"
 
 
+DUMP_BYTES = 64 * 10**6      # --dump-outputs: ceiling on what one dump writes, .npy headers included
+DUMP_SEED = 0xD0             # the fixed row sample of --dump-outputs when all rows would not fit in DUMP_BYTES
+
+
+def dump_outputs(out_dir: str, eng) -> dict:
+    """What the flood leaves its caller, as float64 arrays out_dir/<name>.npy:
+
+    counters.npy  the ra_counters fields in include/ra_engine.h order, totals over the whole run
+    row.npy       the rows dumped: all of them, or a fixed sample (seed DUMP_SEED) when all would pass DUMP_BYTES
+    <field>.npy   each ra_row_state field of those rows, shape (rows,) or (rows, k); the peers' fields as
+                  peer_<field>.npy, one column per member.  Entries RaRowState.key() does not compare (runs past
+                  n_runs, peers past n_members, the cond_reply_* fields while flags bit 1 is clear) are zero, so
+                  two builds compare the way the parity diff does.
+    Every value is an integer below 2^53 (checked), so float64 holds it exactly."""
+    import numpy as np
+    from ra_b200 import abi
+    dt = np.dtype(abi.RaRowState)
+    peer_fields = [f for f in dt["peers"].base.names if not f.startswith("_")]
+    n, m = eng.n_rows, eng.n_members
+    cols = sum(int(np.prod(dt[f].shape)) for f in dt.names if f != "peers") + len(peer_fields) * m
+    k = min(n, (DUMP_BYTES - 2**20) // (8 * cols))       # 1 MiB left for the counters and the .npy headers
+    ids = np.arange(n) if k == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+    rows = np.frombuffer(b"".join(bytes(r) for r in eng.read_rows(ids.tolist())), dtype=dt)
+    out = {"counters": np.array(list(eng.counters().values()), dtype=np.uint64)}
+    out.update((f, rows[f]) for f in dt.names if f != "peers")
+    run_live = np.arange(abi.RA_MAX_RUNS) < rows["n_runs"][:, None]
+    for f in ("run_start", "run_term"):
+        out[f] = np.where(run_live, rows[f], 0)
+    cond_live = (rows["flags"] & 2) != 0
+    for f in ("cond_reply_term", "cond_reply_next_index", "cond_reply_last_index", "cond_reply_last_term"):
+        out[f] = np.where(cond_live, rows[f], 0)
+    peer_live = np.arange(m) < rows["n_members"][:, None]
+    for f in peer_fields:
+        out["peer_" + f] = np.where(peer_live, rows["peers"][f][:, :m], 0)
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in out.items():
+        if a.size and int(a.max()) >= 2**53:
+            raise ValueError("--dump-outputs: %s holds %d, which float64 cannot hold exactly" % (name, int(a.max())))
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a.astype(np.float64))
+        total += os.path.getsize(path)
+    return {"dir": out_dir, "rows": int(k), "of_rows": n, "sample_seed": None if k == n else DUMP_SEED,
+            "files": len(out), "bytes": total}
+
+
 def b_commit(m: int) -> int:
     return (40 + 104 * m) + (m - 1) * (169 + 185) + (128 + 8 * m) + (m - 1) * (145 + 8 * m)
 
@@ -270,6 +316,7 @@ def run_engine(args):
     barrier_sync(world, local)
     clocks = sampler.stop()
     c1 = eng.counters()
+    dump = dump_outputs(args.dump_outputs, eng) if args.dump_outputs else None
     commits = c1["commits"] - c0["commits"]
     events = c1["events"] - c0["events"]
     dropped = c1["msgs_dropped"] - c0["msgs_dropped"]
@@ -410,6 +457,8 @@ def run_engine(args):
         out["latency"] = latency
     if e2e:
         out["e2e"] = e2e
+    if dump:
+        out["dump"] = dump
     if world == 1 and not args.no_cpu:
         out["cpu_baseline"] = cpu_baseline(args, sample_groups=min(G, args.cpu_groups), steps=args.cpu_steps)
     print(json.dumps(out))
@@ -702,7 +751,14 @@ def main():
                     help="skip the keyed entries for the other configs (N=1: 2, 4, 5; N>1: 4 strong-scaled)")
     ap.add_argument("--no-latency", dest="latency", action="store_false", help="skip the per-call latency probe (N=1)")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle replay of every 97th group of this run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the engine's counters and rows as DIR/<name>.npy (float64, "
+                         "at most 64 MB: a fixed sample of the rows when all would not fit); one process only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "engine" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl engine in one process")
     args.faults = None
     if args.config != 3:
         c = CONFIGS[args.config]
