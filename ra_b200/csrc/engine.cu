@@ -145,6 +145,34 @@ __device__ __forceinline__ void flush_ref_counters(const Cols& C, u32 lane, u64 
     }
 }
 
+// Programmatic dependent launch (sm_90+).  A step is a chain of kernels on one stream (step kernel -> general kernel ->
+// next step kernel ...), each reading what the one before wrote.  The two kernels of a step are launched with
+// programmatic stream serialization: the next kernel's CTAs may be scheduled while this one's last CTAs still run
+// (launch_dependents, at the start of every CTA), and grid_dep_wait -- the first statement of both kernels, before any
+// memory access -- blocks until every earlier grid of the stream has completed and its writes are visible.  So the
+// results are those of serial launches; what overlaps is the launch and the CTA ramp-up of the next kernel.
+// (In a kernel launched without the attribute, or behind a copy, grid_dep_wait returns at once.)
+__device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void grid_dep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+#ifdef RA_WARP_TIMELINE
+// Measurement build only (-DRA_WARP_TIMELINE, tools/warp_timeline.py): every warp of a hot-kernel launch that has
+// work writes one record, indexed by its tile, read back through ra_debug_warp_timeline.  The default build has
+// neither the buffer nor the export.
+struct WarpTimeline {
+    u64 t_entry, t_inputs, t_loop, t_exit;    // %globaltimer (ns): entry, per-row inputs landed, event loop done, exit
+    u32 tile;
+    u32 info;                                 // %smid | all lanes leaders << 16 | planes consumed << 24
+    u32 pad[2];
+};
+#define RA_WTL_CAP (1u << 16)                 // warps recorded (tiles beyond are not)
+__device__ WarpTimeline g_wtl[RA_WTL_CAP];
+// the timestamp is taken after `dep` is available: a value the timed phase produced
+__device__ __forceinline__ u64 wtl_now(u32 dep)
+{ u64 t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t) : "r"(dep) : "memory"); return t; }
+__device__ __forceinline__ u32 wtl_smid() { u32 s; asm volatile("mov.u32 %0, %%smid;" : "=r"(s)); return s; }
+#endif
+
 // the hot kernel, once per index width (raft_step.cuh): ra_wide::raft_step_kernel, ra_narrow::raft_step_kernel
 namespace ra_wide {
 #define RA_NARROW_PASS 0
@@ -167,6 +195,8 @@ raft_general_kernel(const __grid_constant__ Cols C, const int cur, const FloodAr
     constexpr int MM = MK_MM(0, TR_RUNTIME);
     __shared__ ulonglong2 s_peers[RA_MAX_MEMBERS * CTA_T + RA_MAX_MEMBERS * CTA_T / 2];   // nm[8][T] then cs[8][T]
     const u32 tid = threadIdx.x, lane = tid & 31u;
+    grid_dep_wait();
+    grid_dep_launch();
     if (*C.abort) return;
     const u32 n = *stall_count;
     for (u32 base = blockIdx.x * CTA_T; base < n; base += gridDim.x * CTA_T) {
@@ -828,6 +858,19 @@ extern "C" int ra_engine_load_query_state(ra_engine* e, const ra_query_state* q,
 extern "C" int ra_engine_read_query_state(ra_engine* e, ra_query_state* q, size_t n)
 { return query_io(e, q, n, false); }
 
+// launch with programmatic stream serialization (see grid_dep_wait): CTA_T threads, `smem` bytes of dynamic shared memory
+template <typename... P, typename... A>
+static cudaError_t launch_chained(void (*k)(P...), u32 grid, size_t smem, cudaStream_t s, A... a)
+{
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(CTA_T); cfg.dynamicSmemBytes = smem; cfg.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, k, a...);
+}
+
 static int launch_step(ra_engine* e, const FloodArgs& F)
 {
     if (e->C.n_shards > 1) {
@@ -845,8 +888,9 @@ static int launch_step(ra_engine* e, const FloodArgs& F)
     u32* cnt = e->d_stall_cnt + (e->steps & 1), *cnt_next = e->d_stall_cnt + ((e->steps + 1) & 1);
     // one specialisation of the hot kernel per (member count, transport): see MK_MM
     const int tr = !e->C.routed ? TR_HOST : (e->C.n_shards > 1 ? (e->C.peer_mode ? TR_PEER : TR_BUCKET) : TR_LOCAL);
-#define LAUNCH_NS(NS, NARROW, MEMB, TRN, FLT) NS::raft_step_kernel<MK_MM(MEMB, TRN), FLT><<<grid, CTA_T, sizeof(StepSmem<MK_MM(MEMB, TRN), NARROW>), e->stream>>>( \
-        e->C, e->cur, F, e->d_stall, cnt, cnt_next)
+    cudaError_t ce = cudaSuccess;
+#define LAUNCH_NS(NS, NARROW, MEMB, TRN, FLT) ce = launch_chained(NS::raft_step_kernel<MK_MM(MEMB, TRN), FLT>, grid, \
+        sizeof(StepSmem<MK_MM(MEMB, TRN), NARROW>), e->stream, e->C, e->cur, F, e->d_stall, cnt, cnt_next)
 #define LAUNCH(MEMB, TRN, FLT) LAUNCH_NS(ra_wide, false, MEMB, TRN, FLT)
 #ifndef RA_NO_NARROW
     // 32-bit index arithmetic for the specialisations that carry the load (exact: rows or records that do not fit
@@ -877,10 +921,11 @@ static int launch_step(ra_engine* e, const FloodArgs& F)
 #undef LAUNCH
 #undef LAUNCH_N
 #undef LAUNCH_NS
-    cudaError_t ce = cudaGetLastError();
+    if (ce == cudaSuccess) ce = cudaGetLastError();
     if (ce != cudaSuccess) return fail(e, ce, "raft_step_kernel");
-    raft_general_kernel<<<e->general_grid, CTA_T, 0, e->stream>>>(e->C, e->cur, F, e->d_stall, cnt);
-    ce = cudaGetLastError();
+    ce = launch_chained(raft_general_kernel, e->general_grid, 0, e->stream, e->C, e->cur, F,
+                        (const StallCtx*)e->d_stall, (const u32*)cnt);
+    if (ce == cudaSuccess) ce = cudaGetLastError();
     if (ce != cudaSuccess) return fail(e, ce, "raft_general_kernel");
     if (e->C.routed) e->cur ^= 1;
     e->steps++;
@@ -1172,6 +1217,29 @@ extern "C" int ra_engine_stall_histogram(ra_engine* e, uint64_t* out128)
     CK(cudaStreamSynchronize(e->stream));
     return RA_OK;
 }
+
+#ifdef RA_WARP_TIMELINE
+// Measurement build only: copies the warp records of the hot-kernel launches since the last clear (48 bytes each,
+// struct WarpTimeline; a warp that had no work writes none) for the first min(tiles, cap) tiles into out, then
+// clears them when `clear` is set.  *n = the number of records copied.  Not part of include/ra_engine.h.
+extern "C" int ra_debug_warp_timeline(ra_engine* e, void* out, size_t cap, size_t* n, int clear)
+{
+    if (!e || !n) return RA_E_INVAL;
+    CK(cudaSetDevice(e->cfg.device));
+    CK(cudaStreamSynchronize(e->stream));
+    size_t k = e->C.tiles < RA_WTL_CAP ? e->C.tiles : RA_WTL_CAP;
+    if (k > cap) k = cap;
+    if (out && k) CK(cudaMemcpyFromSymbol(out, g_wtl, k * sizeof(WarpTimeline)));
+    if (clear) {
+        void* p = nullptr;
+        CK(cudaGetSymbolAddress(&p, g_wtl));
+        CK(cudaMemset(p, 0, sizeof(WarpTimeline) * RA_WTL_CAP));
+    }
+    CK(cudaDeviceSynchronize());
+    *n = k;
+    return RA_OK;
+}
+#endif
 
 extern "C" int ra_engine_set_stream(ra_engine* e, void* cuda_stream)
 {

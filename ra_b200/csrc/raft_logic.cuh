@@ -612,9 +612,9 @@ __device__ __forceinline__ void set_fatal(Member& m, u32 code)
     MT_SET(m.meta, 26, 1, 1);
 }
 
-// out of line on purpose (scalar arguments only, nothing of the member escapes): called from many
-// places, and the hot kernel has to stay small
-__device__ __noinline__ void note_store_raw(ra_note* slot_ptr, u32 row, u32 type, u32 slot, u32 aux, u64 a, u64 b, u64 c)
+// inlined: a leader writes ~3 notes a step, and the out-of-line call (argument moves, CALL / RET) measured slower
+// than the larger code (B200: 0.0798 -> 0.0793 ms per flood step, profiles/r03_ab_explore.txt)
+__device__ __forceinline__ void note_store_raw(ra_note* slot_ptr, u32 row, u32 type, u32 slot, u32 aux, u64 a, u64 b, u64 c)
 {
     ulonglong2* q = reinterpret_cast<ulonglong2*>(slot_ptr);
     q[0] = make_ulonglong2((u64)row | ((u64)(type & 0xff) << 32) | ((u64)(slot & 0xff) << 40) | ((u64)(aux & 0xffff) << 48), a);
@@ -625,8 +625,8 @@ __device__ __forceinline__ void note_store(Member& m, u32 k, u32 type, u32 slot,
     note_store_raw(&m.C->onote[(size_t)k * m.C->rows + m.row], m.row, type, slot, aux, a, b, c);
 }
 
-// a host ("local") event record into tiled plane k; out of line for the same reason
-__device__ __noinline__ void put_local(ulonglong2* loc, u32 tiles, u32 k, u32 row, u32 type, u32 n, u64 term, u64 a, u64 b)
+// a host ("local") event record into tiled plane k; inlined for the same reason
+__device__ __forceinline__ void put_local(ulonglong2* loc, u32 tiles, u32 k, u32 row, u32 type, u32 n, u64 term, u64 a, u64 b)
 {
     ulonglong2* q = loc + rec_word(tiles, k, row, 0);               // RS_PLAIN: head only
     q[0] = make_ulonglong2((u64)type | ((u64)RA_NO_SLOT << 8) | ((u64)RS_PLAIN << 24) | ((u64)(n & 0xffff) << 32), term);

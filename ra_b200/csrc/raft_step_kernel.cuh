@@ -10,6 +10,8 @@ __global__ void __launch_bounds__(CTA_T, RA_STEP_MINB)
 raft_step_kernel(const __grid_constant__ Cols C, const int cur, const FloodArgs F,
                  StallCtx* __restrict__ stall_list, u32* __restrict__ stall_count, u32* __restrict__ stall_count_next)
 {
+    grid_dep_wait();                                            // the step's inputs are the previous kernels' outputs
+    grid_dep_launch();
     extern __shared__ __align__(128) unsigned char smem_raw[];
     typedef StepSmem<MM, RA_NARROW_PASS != 0> Smem;
     Smem& S = *reinterpret_cast<Smem*>(smem_raw);
@@ -27,6 +29,9 @@ raft_step_kernel(const __grid_constant__ Cols C, const int cur, const FloodArgs 
     const u32 wtile = blockIdx.x * WARPS + warp;                 // this warp's record tile
 #endif
     const u32 r = wtile * RT + lane;
+#ifdef RA_WARP_TIMELINE
+    const u64 wtl_t0 = wtl_now(r);
+#endif
     const bool valid = r < C.rows;
     u32 k_events = 0, k_commits = 0, k_applied = 0, k_msgs = 0, k_dropped = 0, k_elect = 0, k_fatal = 0;
     u64 k_ref = 0;
@@ -72,6 +77,10 @@ raft_step_kernel(const __grid_constant__ Cols C, const int cur, const FloodArgs 
     mask_t todo = mask_or_warp(mine);                           // planes still to consume
     const u32 w_tail = __reduce_or_sync(0xffffffffu, my_tail);
     if (!__any_sync(0xffffffffu, work)) return;                 // whole warp idle
+#ifdef RA_WARP_TIMELINE
+    const u64 wtl_t1 = wtl_now(w_tail ^ (u32)ap.y);
+    const bool wtl_leaders = __all_sync(0xffffffffu, valid && MT_ROLE(ap.y) == RA_LEADER);
+#endif
     u64* bars = &S.bars[warp][0];
     if (lane == 0) {
         for (int i = 0; i < NST; i++) mbar_init(&bars[i], 1);
@@ -146,6 +155,9 @@ raft_step_kernel(const __grid_constant__ Cols C, const int cur, const FloodArgs 
         if (++st == NST) { st = 0; par ^= 1u; }
         __syncwarp();                                           // every lane is done with the slot
     }
+#ifdef RA_WARP_TIMELINE
+    const u64 wtl_t2 = wtl_now(n_done);
+#endif
     const u32 rem_mbox = (u32)(rem & (((mask_t)1 << (NPM - 1) << 1) - 1)), rem_loc = (u32)(rem >> (NPM - 1) >> 1);
 
     if (work) {
@@ -176,6 +188,14 @@ raft_step_kernel(const __grid_constant__ Cols C, const int cur, const FloodArgs 
     }
     flush_counters(C, lane, k_events, k_commits, k_applied, k_msgs, k_dropped, k_elect, k_fatal);
     flush_ref_counters(C, lane, k_ref);
+#ifdef RA_WARP_TIMELINE
+    const u64 wtl_t3 = wtl_now(lane);
+    if (lane == 0 && wtile < RA_WTL_CAP) {
+        WarpTimeline& w = g_wtl[wtile];
+        w.t_entry = wtl_t0; w.t_inputs = wtl_t1; w.t_loop = wtl_t2; w.t_exit = wtl_t3;
+        w.tile = wtile; w.info = (wtl_smid() & 0xffffu) | ((wtl_leaders ? 1u : 0u) << 16) | ((n_done & 0xffu) << 24);
+    }
+#endif
 }
 
 #undef RA_STEP_MINB
